@@ -7,6 +7,10 @@ weights.  One "step" = one batch of 32 images through the whole chain.
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # B200 arm (prints ONE JSON line)
     python bench.py --impl reference [--steps K] [--warmup W]      # the reference's CPU implementation of the same chain
+    python bench.py --steps K --dump-outputs DIR                   # also writes what the last of the K timed steps returned
+
+The inputs and weights are seeded, so two runs with the same arguments see the same data and their --dump-outputs files compare
+output for output.  The bench writes nothing into the source tree; its scratch files go to the temporary directory.
 
 N > 1: launched by torch.distributed.run, one rank per GPU; the inference path shards by image with no
 data-path collective (replicas), so scaling is "weak" and `value` is the whole-job rate
@@ -389,6 +393,40 @@ def timed_steps(pipe, steps, warmup, slots, cur, barrier, world, device):
     return ms
 
 
+def dump_outputs(pipe, slot, out_dir, budget=64 << 20):
+    """Writes what the caller of the timed path received from its last step (input slot `slot`) as out_dir/<name>.npy: the decoded
+    head (feature, iou, yx_min, yx_max, prob) and every image's detections in the form detect.postprocess returns them (keep_iou,
+    det_yx_min, det_yx_max, det_cls, det_score), concatenated over images; n_keep / n_det per image split them.  Float arrays are
+    float32, counts and classes float64 (exact).  Images are taken in batch order while the files fit in `budget` bytes."""
+    import numpy as np
+    import torch
+    host = pipe.fetch(slot)
+    torch.cuda.synchronize()
+    dense = {k: pipe.out[slot][k].float().cpu().numpy() for k in ('feature', 'iou', 'yx_min', 'yx_max', 'prob')}
+    parts = {k: [] for k in ('n_keep', 'n_det', 'keep_iou', 'det_yx_min', 'det_yx_max', 'det_cls', 'det_score')}
+    used = 128 * (len(dense) + len(parts))         # .npy headers
+    for bi in range(pipe.batch):
+        d = pipe.detections(host, bi)
+        iou, yx_min, yx_max, cls, score = (torch.zeros(0), torch.zeros(0, 2), torch.zeros(0, 2), torch.zeros(0), torch.zeros(0)) if d is None else d
+        size = sum(v[bi].nbytes for v in dense.values()) + 8 * (2 + iou.numel() + 6 * cls.numel())
+        if used + size > budget:
+            break
+        used += size
+        parts['n_keep'].append(np.array([iou.numel()], np.float64))
+        parts['n_det'].append(np.array([cls.numel()], np.float64))
+        parts['keep_iou'].append(iou.float().numpy())
+        parts['det_yx_min'].append(yx_min.float().numpy())
+        parts['det_yx_max'].append(yx_max.float().numpy())
+        parts['det_cls'].append(cls.double().numpy())
+        parts['det_score'].append(score.float().numpy())
+    n = len(parts['n_keep'])
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in dense.items():
+        np.save(os.path.join(out_dir, k + '.npy'), v[:n])
+    for k, v in parts.items():
+        np.save(os.path.join(out_dir, k + '.npy'), np.concatenate(v))
+
+
 def mobilenet_record(args, device, peaks):
     """BASELINE configs[4]: MobileNet backbone 416x416 batch-32 + decode + filter + NMS through the plugin surface, one CUDA graph."""
     import torch
@@ -594,6 +632,9 @@ def run_b200(args):
     t_wall = time.perf_counter()
     ms = timed_steps(pipe, args.steps, args.warmup, slots, cur, barrier, world, device)
     wall_ms = (time.perf_counter() - t_wall) * 1e3
+    if args.dump_outputs and rank == 0:
+        # now: the pipelines timed next share the engine's per-lane activation plans, where the head feature lives
+        dump_outputs(pipe, (args.steps - 1) % slots, args.dump_outputs)
     graph_launches = pipe.launches_per_run * args.steps
     value = world * B * args.steps / (ms / 1e3)
 
@@ -683,6 +724,7 @@ def run_b200(args):
                     share_of_step=share, step_ms=step1_ms,
                     how='share = conv CUDA-event time / all kernels\' CUDA-event time in an instrumented eager pass of this run; us_per_launch = share x one_lane.ms_per_step / 22',
                     eager_event_sum=dict(conv_ms=prof['conv_ms'], all_kernels_ms=prof['kernels_ms'], note='isolated CUDA events add ~2-4 us per kernel: only the ratio is used'),
+                    layers=prof['layers'],
                     whole_step_two_lanes=dict(tflops=(B * GFLOP_PER_IMAGE_416 / 1e3) / (graph_step_ms / 1e3),
                                               frac=(B * GFLOP_PER_IMAGE_416 / 1e3) / (graph_step_ms / 1e3) / peaks['tflops']))
     # HBM-bound kernels of the step: algorithmic bytes (SURVEY 8d, fp16 activations inside the backbone) / their slice of the one-lane step
@@ -702,9 +744,6 @@ def run_b200(args):
             us = rec['us_per_step'] / (prof['kernels_ms'] * 1e3) * step1_ms * 1e3
             gbs = nbytes / (us * 1e-6) / 1e9
             hbm_kernels[name] = dict(us=us, alg_bytes=nbytes, achieved_gbs=gbs, frac_of_hbm_peak=gbs / peaks['hbm'])
-    os.makedirs(os.path.join(ROOT, 'gpurun_out'), exist_ok=True)
-    with open(os.path.join(ROOT, 'gpurun_out', 'bench_layers.json'), 'w') as f:
-        json.dump(dict(prof, graph_step_ms=graph_step_ms, one_lane_step_ms=step1_ms, value=value), f, indent=1)
 
     mobilenet = None
     if not args.no_mobilenet:
@@ -928,7 +967,11 @@ def main():
     ap.add_argument('--cpu-budget', type=float, default=150.0, help='reference arm: seconds of CPU work for the whole run')
     ap.add_argument('--keep-features', type=int, default=0, help=argparse.SUPPRESS)
     ap.add_argument('--features-out', default=None, help=argparse.SUPPRESS)
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the arrays the last timed step returned (detections, decoded head) as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != 'b200' or args.mode != 'infer'):
+        ap.error('--dump-outputs applies to the B200 inference arm')
     if args.impl == 'reference':
         # the reference moves tensors to a GPU whenever it sees one (utils/__init__.py:104-111); this arm is its CPU path
         os.environ['CUDA_VISIBLE_DEVICES'] = ''

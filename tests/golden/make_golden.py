@@ -111,13 +111,16 @@ def main():
                         **{'act_' + k: v.numpy() for k, v in outs.items()})
 
     # ---- 2. backbone at 416x416: feature + per-layer checksums ------------------------------
+    # evaluated in float64 and stored rounded to float32: fp32 sums over 23 layers differ from CPU to CPU (vector ISA, thread
+    # count) by more than the test's tolerances, so the fixture holds the exact values, which the test's float64 oracle meets anywhere
     outs.clear()
     x416 = O.synth_images(1, 416, 416, seed=0)
     with torch.no_grad():
-        f416 = dnn(x416)
-    np.savez_compressed(os.path.join(HERE, 'darknet_416.npz'), feature=f416.numpy(),
-                        **{'absmean_' + k: np.float64(v.double().abs().mean().item()) for k, v in outs.items()},
-                        **{'head_' + k: v.flatten()[:64].numpy() for k, v in outs.items()})
+        f416 = dnn.double()(x416.double())
+    dnn.float()
+    np.savez_compressed(os.path.join(HERE, 'darknet_416.npz'), feature=f416.float().numpy(),
+                        **{'absmean_' + k: np.float64(v.abs().mean().item()) for k, v in outs.items()},
+                        **{'head_' + k: v.flatten()[:64].float().numpy() for k, v in outs.items()})
     for h in hooks:
         h.remove()
 

@@ -35,10 +35,16 @@ def test_backbone_64_every_layer(golden_dir):
     np.testing.assert_allclose(f.numpy(), g['feature'], rtol=0, atol=2e-5 * np.abs(g['feature']).max())
 
 
+def _double(sd):
+    return {k: v.double() if v.is_floating_point() else v for k, v in sd.items()}
+
+
 def test_backbone_416_feature(golden_dir):
+    """Both sides in float64 (the fixture rounded to float32): fp32 sums over 23 layers depend on the CPU's vector ISA and thread
+    count by more than these tolerances."""
     g = load(golden_dir, 'darknet_416.npz')
-    sd = O.make_state_dict(0)
-    x = O.synth_images(1, 416, 416, seed=0)
+    sd = _double(O.make_state_dict(0))
+    x = O.synth_images(1, 416, 416, seed=0).double()
     collect = {}
     with torch.no_grad():
         f = O.darknet_forward(sd, x, collect=collect)
@@ -230,16 +236,15 @@ def test_resize_oracle_matches_cv2_golden(golden_dir):
         out = O.resize_u8(O.synth_frame(seed, h0, w0), h, w)
         assert out.shape == (h, w, 3)
         assert hashlib.sha256(out.tobytes()).digest() == g['case%d_sha' % seed].tobytes(), seed
-    jpg = '/root/reference/image.jpg'
-    if os.path.exists(jpg):                                   # build container only: the reference's own sample image
-        import cv2
-        img = cv2.imread(jpg)
-        if hashlib.sha256(img.tobytes()).digest() == g['jpg_src_sha'].tobytes():
-            r, a, b = O.rescale_label(img, g['jpg_yx_min_in'].copy(), g['jpg_yx_max_in'].copy(), 416, 416)
-            assert hashlib.sha256(r.tobytes()).digest() == g['jpg_sha_bgr'].tobytes()
-            assert hashlib.sha256(r[..., ::-1].tobytes()).digest() == g['jpg_sha_rgb'].tobytes()
-            assert np.array_equal(a, g['jpg_yx_min']) and np.array_equal(b, g['jpg_yx_max'])
-            assert np.array_equal(r[100:132, 200:232], g['jpg_crop'])
+    # the reference's own sample image (tests/golden/image.jpg), decoded as the golden script decoded it
+    import cv2
+    img = cv2.imread(os.path.join(golden_dir, 'image.jpg'))
+    assert hashlib.sha256(img.tobytes()).digest() == g['jpg_src_sha'].tobytes()
+    r, a, b = O.rescale_label(img, g['jpg_yx_min_in'].copy(), g['jpg_yx_max_in'].copy(), 416, 416)
+    assert hashlib.sha256(r.tobytes()).digest() == g['jpg_sha_bgr'].tobytes()
+    assert hashlib.sha256(r[..., ::-1].tobytes()).digest() == g['jpg_sha_rgb'].tobytes()
+    assert np.array_equal(a, g['jpg_yx_min']) and np.array_equal(b, g['jpg_yx_max'])
+    assert np.array_equal(r[100:132, 200:232], g['jpg_crop'])
 
 
 @pytest.mark.parametrize('tag', list('abcd'))
@@ -311,13 +316,14 @@ def test_training_step_oracle_matches_executed_reference(golden_dir):
 def test_c1_single_image_chain_oracle_matches_executed_reference(golden_dir):
     """BASELINE configs[0]: the reference's detect.py chain on its own image.jpg (resize, BGR2RGB, ToTensor, Darknet-19,
     decode, softmax, postprocess with detect/fix = 1), executed by tests/golden/make_golden_c1.py, against the oracle on the
-    stored 416x416 RGB network input: feature map, and the detection tuple with exact class / box-index agreement."""
+    stored 416x416 RGB network input: feature map, and the detection tuple with exact class / box-index agreement.  The backbone runs
+    in float64 on both sides, its feature rounded to float32 for the rest of the chain (as in test_backbone_416_feature)."""
     g = load(golden_dir, 'c1_image.npz')
-    sd = O.make_state_dict(seed=0)
+    sd = _double(O.make_state_dict(seed=0))
     anchors = O.anchors_yolo_voc()
-    x = torch.from_numpy(g['rgb'].transpose(2, 0, 1).copy()).float().div(255).unsqueeze(0)
+    x = torch.from_numpy(g['rgb'].transpose(2, 0, 1).copy()).float().div(255).unsqueeze(0).double()
     with torch.no_grad():
-        feature = O.darknet_forward(sd, x)
+        feature = O.darknet_forward(sd, x).float()
         pred = O.decode(feature, anchors)
         prob = O.class_prob(pred)
         res = O.postprocess(pred['iou'][0].reshape(-1), pred['yx_min'][0].reshape(-1, 2), pred['yx_max'][0].reshape(-1, 2),
@@ -329,11 +335,9 @@ def test_c1_single_image_chain_oracle_matches_executed_reference(golden_dir):
         np.testing.assert_allclose(res[0].numpy(), g['det_iou'], rtol=1e-5, atol=1e-7)
         np.testing.assert_allclose(res[1].numpy(), g['det_yx_min'], rtol=1e-5, atol=1e-5)
         np.testing.assert_allclose(res[4].numpy(), g['det_score'], rtol=1e-5, atol=1e-8)
-    # the stored network input is what the oracle's cv2-exact resize produces from the reference's sample image, if present
-    jpg = '/root/reference/image.jpg'
-    if os.path.exists(jpg):
-        import cv2
-        assert np.array_equal(O.resize_u8(cv2.imread(jpg), 416, 416)[..., ::-1], g['rgb'])
+    # the stored network input is what the oracle's cv2-exact resize produces from the reference's sample image
+    import cv2
+    assert np.array_equal(O.resize_u8(cv2.imread(os.path.join(golden_dir, 'image.jpg')), 416, 416)[..., ::-1], g['rgb'])
 
 
 def test_c2_batch32_oracle_matches_executed_reference(golden_dir):

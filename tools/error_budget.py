@@ -6,8 +6,8 @@ reference's 1e-3 contract needs ~3/4 of the roundings removed: b200.engine.STRIC
 
     python tools/error_budget.py
 """
-import sys, time, torch, torch.nn.functional as F
-sys.path.insert(0, '/root/repo')
+import os, sys, time, torch, torch.nn.functional as F
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from oracle import yolo2_oracle as O
 torch.set_num_threads(8)
 sd = O.make_state_dict(0)

@@ -6,8 +6,8 @@ test (tests/test_gpu_parity.py: C3) asserts losses / statistics and the per-laye
 
     python tools/train_error_budget.py 8 416     # batch, size  ->  profiles/r02_train_error_budget.txt
 """
-import sys, time, torch, torch.nn.functional as F
-sys.path.insert(0, '/root/repo')
+import os, sys, time, torch, torch.nn.functional as F
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from oracle import yolo2_oracle as O
 torch.set_num_threads(8)
 sd = O.make_state_dict(0)
