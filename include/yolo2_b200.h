@@ -274,6 +274,20 @@ int yb_warp_affine_u8(const void* src, int src_h, int src_w, void* dst, int dst_
  * value / 255.  Only the training path needs the fp32 image (inference reads the uint8 frames in the first conv kernel). */
 int yb_totensor_u8(const void* src_nhwc_u8, float* dst_nchw_f32, int batch, int height, int width, yb_stream_t stream);
 
+/* Photometric training augmentations of transform/image.py:32-99 (RandomBlur, BGR2HSV, RandomHue, RandomSaturation, RandomBrightness,
+ * HSV2RGB, RandomGamma; applied per resized image at utils/data.py:121) for a batch of same-size uint8 HWC frames [B,height,width,3] in
+ * one launch, each image with its own parameters.  Stages in this order, each optional:
+ *   blur_k  int[B][2] (kx, ky), 1 <= k <= 15 (NULL = no blur): cv2.blur(img, (kx, ky)), BORDER_REFLECT_101; src and dst must not alias
+ *   to_hsv  cv2 COLOR_BGR2HSV, 8-bit (H in 0..179), bit-exact
+ *   lut_hsv uint8[B][3][256] (NULL = identity): per-image, per-channel table (hue / saturation / brightness, composed on the host)
+ *   to_rgb  cv2 COLOR_HSV2RGB, 8-bit, bit-exact
+ *   lut_out uint8[B][3][256] (NULL = identity): per-image, per-channel table (gamma)
+ * All pointers are device pointers.  The blur is cv2's arithmetic with one intended difference: an area-2 window of two 255s gives 255
+ * (cv2 wraps it to 0 in its scalar tail loop, so its result depends on the row width).  Images whose (kx, ky) lie outside 1..15 are
+ * left unwritten; the Python wrappers reject such draws before the launch. */
+int yb_photometric_u8(const void* src, void* dst, int batch, int height, int width, const int* blur_k, int to_hsv, const unsigned char* lut_hsv,
+                      int to_rgb, const unsigned char* lut_out, yb_stream_t stream);
+
 /* ---- evaluation matching (SURVEY 8f rank 3; eval.py:57-75 `_matching`/`matching`, called per image and class at eval.py:210-216) ----
  * Segmented batch: image i owns detections [det_off[i], det_off[i+1]) (descending score within the image, as postprocess returns
  * them) and ground-truth boxes [gt_off[i], gt_off[i+1]); boxes are (y, x) float pairs, classes int32.  tp[d] = 1 iff detection d's

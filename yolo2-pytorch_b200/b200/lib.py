@@ -60,6 +60,7 @@ SIGNATURES = {
     'yb_resize_aug_batch_u8': [P, P, P, P, P, P, P, c_int, c_int, c_int, c_int, P, P, c_int, P],
     'yb_warp_affine_u8': [P, c_int, c_int, P, c_int, c_int, ctypes.POINTER(ctypes.c_double * 6), ctypes.POINTER(c_int * 3), P],
     'yb_totensor_u8': [P, P, c_int, c_int, c_int, P],
+    'yb_photometric_u8': [P, P, c_int, c_int, c_int, P, c_int, P, c_int, P, P],
     'yb_eval_match': [P, P, P, P, P, P, P, P, c_int, c_int, c_int, c_float, c_float, P, P],
     'yb_mb_conv0_raw_fwd': [P, P, P, c_int, c_int, c_int, P],
     'yb_mb_conv0_split_fwd': [P, P, P, P, P, c_int, c_int, c_int, P],

@@ -102,6 +102,7 @@ int totensor_u8(const void*, float*, int, int, int, cudaStream_t);
 int warp_affine_u8(const void*, int, int, void*, int, int, const double*, const int*, cudaStream_t);
 int resize_aug_batch_u8(const void*, const long long*, const int*, const int*, const float*, const unsigned char*, void*, int, int, int, int, float*, float*,
                         int, cudaStream_t);
+int photometric_u8(const void*, void*, int, int, int, const int*, int, const unsigned char*, int, const unsigned char*, cudaStream_t);
 int eval_match(const float*, const float*, const int*, const int*, const float*, const float*, const int*, const int*, int, int, int, float, float,
                unsigned char*, cudaStream_t);
 int unpack_wgrad(const float*, float*, int, int, int, float, cudaStream_t);
@@ -359,6 +360,11 @@ int yb_warp_affine_u8(const void* src, int src_h, int src_w, void* dst, int dst_
 
 int yb_totensor_u8(const void* src_nhwc_u8, float* dst_nchw_f32, int batch, int height, int width, yb_stream_t stream) {
   return yb::totensor_u8(src_nhwc_u8, dst_nchw_f32, batch, height, width, S(stream));
+}
+
+int yb_photometric_u8(const void* src, void* dst, int batch, int height, int width, const int* blur_k, int to_hsv, const unsigned char* lut_hsv,
+                      int to_rgb, const unsigned char* lut_out, yb_stream_t stream) {
+  return yb::photometric_u8(src, dst, batch, height, width, blur_k, to_hsv, lut_hsv, to_rgb, lut_out, S(stream));
 }
 
 int yb_eval_match(const float* det_yx_min, const float* det_yx_max, const int* det_cls, const int* det_off, const float* gt_yx_min,

@@ -4,7 +4,12 @@
 frames in one launch -- optionally through the horizontal flip and the random-crop window of the reference's training pipeline
 (`transform.augmentation.flip_horizontally`, `transform.resize.label.random_crop`), which are index transforms on the source of the same
 resize; `transform.augmentation.random_rotate` / `Rotator` and `transform.resize.image.fixed` (shrinking) run cv2.warpAffine's bilinear path in
-one kernel.  The photometric augmentations of `transform/image.py` (blur / hue / saturation / brightness / gamma) are not part of this build."""
+one kernel.  The photometric augmentations of `transform/image.py` (`RandomBlur`, `BGR2HSV`, `RandomHue`, `RandomSaturation`,
+`RandomBrightness`, `HSV2RGB`, `RandomGamma`) run as one batched kernel (`transform.image.apply_chain`, yb_photometric_u8); `get_transform`
+builds the reference's `image_train` chain from its config line, and `utils.data.Collate(..., transform_image=...)` applies it to the
+resized batch."""
+import inspect
+
 import torch
 
 from b200 import ops as _ops
@@ -65,3 +70,36 @@ def to_tensor(frames_u8):
     out = torch.empty(b, 3, h, w, dtype=torch.float32, device=frames_u8.device)
     _ops.call('yb_totensor_u8', frames_u8, out, b, h, w)
     return out
+
+
+class Compose(object):
+    """torchvision.transforms.Compose: apply `transforms` in order.  A chain made only of photometric `transform.image` ops runs
+    through `transform.image.apply_chain` (the reference's draw order, one launch per run of ascending kernel stages)."""
+
+    def __init__(self, transforms):
+        self.transforms = list(transforms)
+
+    def __call__(self, image):
+        from transform import image as _image
+        if self.transforms and all(isinstance(t, _image.Photometric) for t in self.transforms):
+            return _image.apply_chain(self.transforms, image)
+        for t in self.transforms:
+            image = t(image)
+        return image
+
+
+def parse_transform(config, method):
+    """A dotted name -> `cls(config)` when the constructor takes one argument, `cls()` otherwise (reference transform/__init__.py:25-34);
+    anything else is returned as is."""
+    if isinstance(method, str):
+        import utils
+        attr = utils.parse_attr(method)
+        if len(inspect.signature(attr).parameters) == 1:
+            return attr(config)
+        return attr()
+    return method
+
+
+def get_transform(config, sequence, compose=Compose):
+    """e.g. get_transform(config, config.get('transform', 'image_train').split()) (reference transform/__init__.py:37-38)."""
+    return compose([parse_transform(config, method) for method in sequence])

@@ -56,14 +56,30 @@ class Collate(object):
                  into the first conv kernel)
         yx_min / yx_max float32 [B, G, 2] in pixels of the resized image, zero-padded (train.norm_data scales to grid units)
         cls int64 [B, G], difficult uint8 [B, G], size int64 [B, 2] (original sizes), height, width
-    The reference's `resize` config choice maps to `rescale` (the default, transform/resize/label.py:25-31)."""
+    The reference's `resize` config choice maps to `rescale` (the default, transform/resize/label.py:25-31).
+    `transform_image` is the reference's keyword (utils/data.py:94,121), typically
+    `transform.get_transform(config, config.get('transform', 'image_train').split())`.  None or exactly [BGR2RGB] keeps the swap fused
+    into the resize.  Otherwise the resize runs without the swap (`image_train` replaces BGR2RGB, as in the reference) and the chain
+    -- photometric `transform.image` ops -- runs on the whole batch: draws image by image in chain order, as the reference's loop
+    makes them, and one launch per run of ops that fits the kernel's stage order (the full reference chain is one launch)."""
 
-    def __init__(self, sizes, maintain=1, seed=None, bgr2rgb=True):
+    def __init__(self, sizes, maintain=1, seed=None, bgr2rgb=True, transform_image=None):
         self.schedule = SizeSchedule(sizes, maintain, seed)
         self.bgr2rgb = bgr2rgb
+        self.chain = None
+        if transform_image is not None:
+            from transform import image as _image
+            if isinstance(transform_image, _image.Photometric):
+                chain = [transform_image]
+            else:
+                chain = list(getattr(transform_image, 'transforms', transform_image))
+            if not (len(chain) == 1 and isinstance(chain[0], _image.BGR2RGB)):
+                _image.split_chain(chain)          # TypeError for anything but photometric ops
+                self.bgr2rgb = False
+                self.chain = chain
 
     def __call__(self, batch):
-        import transform
+        import transform.image
         height, width = self.schedule.next_size()
         dim = max(max(len(d['cls']) for d in batch), 1)
         frames, rows = [], []
@@ -80,6 +96,8 @@ class Collate(object):
         yx_min = torch.from_numpy(np.stack([r['yx_min'] for r in rows]).astype(np.float32))
         yx_max = torch.from_numpy(np.stack([r['yx_max'] for r in rows]).astype(np.float32))
         tensor, yx_min, yx_max = transform.resize_batch(frames, height, width, bgr2rgb=self.bgr2rgb, yx_min=yx_min, yx_max=yx_max)
+        if self.chain is not None:
+            tensor = transform.image.apply_chain(self.chain, tensor)
         dev = tensor.device
         return dict(tensor=tensor, yx_min=yx_min, yx_max=yx_max,
                     cls=torch.from_numpy(np.stack([np.asarray(r['cls']) for r in rows]).astype(np.int64)).to(dev),
