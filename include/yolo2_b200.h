@@ -315,6 +315,22 @@ int yb_maxpool3x3_s2_f16(const void* x, void* y, int batch, int height, int widt
 int yb_subsample2_f16(const void* x, void* y, int batch, int height, int width, int channels, yb_stream_t stream);
 int yb_add_relu_f16(const void* a, const void* b, void* out, long long count, yb_stream_t stream);
 
+/* ---- DenseNet plugin (model/densenet.py:29-117, torchvision's _DenseLayer / _Transition), inference -------------------------------------
+ * The stem is yb_stem7x7_bn_relu_fwd (64 outputs: densenet121/169/201) or yb_stem7x7_96_bn_relu_fwd (96 outputs: densenet161), same contract.
+ * yb_maxpool3x3_s2_strided_f16: yb_maxpool3x3_s2_f16 writing channels [y_ch_off, y_ch_off + channels) of an fp16 NHWC output of pitch y_ld (the first
+ * dense block's concatenation buffer); yb_maxpool3x3_s2_f16 is its y_ld = channels, y_ch_off = 0 case.
+ * yb_bn_relu_f16: y[p, c] = fp16(max(fmaf(x[p, c], scale[c], shift[c]), 0)) for c < channels, 0 for channels <= c < channels_padded; x and y fp16 with
+ * pixel pitches x_ld / y_ld.  channels, channels_padded, x_ld, y_ld multiples of 8, pointers 16B aligned, else YB_ERR_BAD_ARG.
+ * yb_bn_relu_avgpool2x2_f16: y[b, oy, ox, c] = fp16(0.25 * sum over rows 2oy..2oy+1, columns 2ox..2ox+1 of relu(fmaf(x, scale, shift))), summed in
+ * fp32; x [B,H,W] of pitch x_ld, y contiguous [B, H/2, W/2, channels] (odd sizes floor, as AvgPool2d(2, 2)). */
+int yb_stem7x7_96_bn_relu_fwd(const float* x_nchw, const float* w_oihw, const float* scale, const float* shift, void* y_nhwc_f16, int batch, int height,
+                              int width, yb_stream_t stream);
+int yb_maxpool3x3_s2_strided_f16(const void* x, void* y, int batch, int height, int width, int channels, int y_ld, int y_ch_off, yb_stream_t stream);
+int yb_bn_relu_f16(const void* x, int x_ld, const float* scale, const float* shift, void* y, int y_ld, long long pixels, int channels, int channels_padded,
+                   yb_stream_t stream);
+int yb_bn_relu_avgpool2x2_f16(const void* x, int x_ld, const float* scale, const float* shift, void* y, int batch, int height, int width, int channels,
+                              yb_stream_t stream);
+
 /* Training of the MobileNet plugin: what torch autograd does for conv_bn / conv_dw (model/mobilenet.py:25-38).  The raw forms return the conv
  * output before BatchNorm / ReLU (train-mode statistics come from yb_bn_stats / yb_bn_finalize, the activation from yb_bn_act_apply with slope 0);
  * height / width are always those of the conv INPUT.  dgrad: da fp16 [B,H,W,C] from dz fp16 [B,H/stride,W/stride,C]; wgrad: dw fp32 [C][9]

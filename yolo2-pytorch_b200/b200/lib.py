@@ -73,6 +73,10 @@ SIGNATURES = {
     'yb_maxpool3x3_s2_f16': [P, P, c_int, c_int, c_int, c_int, P],
     'yb_subsample2_f16': [P, P, c_int, c_int, c_int, c_int, P],
     'yb_add_relu_f16': [P, P, P, c_longlong, P],
+    'yb_stem7x7_96_bn_relu_fwd': [P, P, P, P, P, c_int, c_int, c_int, P],
+    'yb_maxpool3x3_s2_strided_f16': [P, P, c_int, c_int, c_int, c_int, c_int, c_int, P],
+    'yb_bn_relu_f16': [P, c_int, P, P, P, c_int, c_longlong, c_int, c_int, P],
+    'yb_bn_relu_avgpool2x2_f16': [P, c_int, P, P, P, c_int, c_int, c_int, c_int, P],
     'yb_comm_version': [ctypes.POINTER(c_int)],
     'yb_comm_unique_id': [P],
     'yb_comm_init': [ctypes.POINTER(P), c_int, P, c_int],

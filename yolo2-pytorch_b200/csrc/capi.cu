@@ -109,7 +109,11 @@ int unpack_wgrad(const float*, float*, int, int, int, float, cudaStream_t);
 int grad_guard(float*, long long, float*, int, cudaStream_t);
 int conv_wgrad_forward(const void*, const void*, float*, int, int, int, int, int, int, int, int, cudaStream_t);
 int stem7x7(const float*, const float*, const float*, const float*, void*, int, int, int, cudaStream_t);
+int stem7x7_96(const float*, const float*, const float*, const float*, void*, int, int, int, cudaStream_t);
 int maxpool3x3_s2(const void*, void*, int, int, int, int, cudaStream_t);
+int maxpool3x3_s2_strided(const void*, void*, int, int, int, int, int, int, cudaStream_t);
+int bn_relu(const void*, int, const float*, const float*, void*, int, long long, int, int, cudaStream_t);
+int bn_relu_avgpool2x2(const void*, int, const float*, const float*, void*, int, int, int, int, cudaStream_t);
 int subsample2(const void*, void*, int, int, int, int, cudaStream_t);
 int add_relu(const void*, const void*, void*, long long, cudaStream_t);
 int comm_version(int*);
@@ -421,6 +425,25 @@ int yb_stem7x7_bn_relu_fwd(const float* x_nchw, const float* w_oihw, const float
 
 int yb_maxpool3x3_s2_f16(const void* x, void* y, int batch, int height, int width, int channels, yb_stream_t stream) {
   return yb::maxpool3x3_s2(x, y, batch, height, width, channels, S(stream));
+}
+
+int yb_stem7x7_96_bn_relu_fwd(const float* x_nchw, const float* w_oihw, const float* scale, const float* shift, void* y_nhwc_f16, int batch, int height,
+                              int width, yb_stream_t stream) {
+  return yb::stem7x7_96(x_nchw, w_oihw, scale, shift, y_nhwc_f16, batch, height, width, S(stream));
+}
+
+int yb_maxpool3x3_s2_strided_f16(const void* x, void* y, int batch, int height, int width, int channels, int y_ld, int y_ch_off, yb_stream_t stream) {
+  return yb::maxpool3x3_s2_strided(x, y, batch, height, width, channels, y_ld, y_ch_off, S(stream));
+}
+
+int yb_bn_relu_f16(const void* x, int x_ld, const float* scale, const float* shift, void* y, int y_ld, long long pixels, int channels, int channels_padded,
+                   yb_stream_t stream) {
+  return yb::bn_relu(x, x_ld, scale, shift, y, y_ld, pixels, channels, channels_padded, S(stream));
+}
+
+int yb_bn_relu_avgpool2x2_f16(const void* x, int x_ld, const float* scale, const float* shift, void* y, int batch, int height, int width, int channels,
+                              yb_stream_t stream) {
+  return yb::bn_relu_avgpool2x2(x, x_ld, scale, shift, y, batch, height, width, channels, S(stream));
 }
 
 int yb_subsample2_f16(const void* x, void* y, int batch, int height, int width, int channels, yb_stream_t stream) {
